@@ -49,6 +49,8 @@ def _args():
     p.add_argument("--nlayers", type=int, default=0, help="debug only: override depth (result is flagged invalid)")
     p.add_argument("--trace", default="", help="with --profile: also export the chrome trace of the 2 profiled steps")
     p.add_argument("--profile", default="", help="write a per-kernel device-time table of 2 extra steps to this path")
+    p.add_argument("--dump-outputs", default="", metavar="DIR",
+                   help="after the device-timed steps, write what the last of them computed to DIR/<name>.npy")
     return p.parse_args()
 
 
@@ -60,6 +62,34 @@ def bench_config(model, global_batch, seq, parallelism, ac):
     return {"model": model, "global_batch": global_batch, "seq_len": seq, "parallelism": parallelism,
             "selective_ac": str(ac), "data_stream": "get_dummy_loader (arange windows mod vocab, label == input)",
             "l2": "per-step working set (>=13.5 GB of weights+activations) >> 126 MB L2; no explicit flush"}
+
+
+DUMP_SAMPLE = 4096   # values kept per parameter tensor by --dump-outputs
+
+
+def dump_outputs(out_dir, eng, loss, grad_norm, rank):
+    """Write what one training step returned and updated, as float32 ``.npy`` files: ``loss``, ``grad_norm`` and, for every
+    parameter, ``param.<name>`` = the fp32 master weights after the optimizer step at DUMP_SAMPLE positions drawn from a
+    fixed seed (all of a smaller tensor).  Same arguments, same inputs: two builds can be compared file by file.  The step
+    is not bitwise reproducible (some kernels accumulate with atomics), so compare with a tolerance: two runs of one build
+    on a B200 (1000 W) differed by 1e-4 relative in the loss and 3e-6 absolute in the weights.  Every rank takes part in
+    the parameter gathers; rank 0 writes."""
+    import numpy as np
+    import torch
+
+    arrays = {"loss": loss, "grad_norm": grad_norm}
+    gen = torch.Generator().manual_seed(0)
+    for u in eng.units:
+        flat = eng.gather_unit_full(u, "master")
+        for name, v in eng.named_unit_views(u, flat):
+            v = v.reshape(-1)
+            if v.numel() > DUMP_SAMPLE:
+                v = v[torch.randint(v.numel(), (DUMP_SAMPLE,), generator=gen).sort().values.to(v.device)]
+            arrays[f"param.{name}"] = v
+    if rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        for name, t in arrays.items():
+            np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 class ClockSampler:
@@ -233,6 +263,8 @@ def run_ours(a):
     fallbacks = CK.fallback_count()
     peak_alloc = torch.cuda.max_memory_allocated(dev)   # train() below resets the peak counters at its report step
     loss_timed = float(loss_sum) / a.steps      # mean loss of steps W+1 .. W+K (what the reference arm prints too)
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, eng, loss, gn, rank)
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)

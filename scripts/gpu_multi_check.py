@@ -1,7 +1,8 @@
 """Multi-GPU check (torchrun, one rank per GPU): fused NVLink collectives vs c10d/NCCL.
  1. raw kernels: p2p all-gather / pull reduce-scatter on 7B-block-sized buffers, numerics + bus bandwidth
  2. engine: same model/data trained with collective_impl=fused and =torch must agree
-Writes gpurun_out/multi_<world>.json from rank 0."""
+Rank 0 prints the results as one JSON line and, given a second argument, also writes them to that file:
+    python -m torch.distributed.run --nproc-per-node N scripts/gpu_multi_check.py all [OUT.json]"""
 import json
 import os
 import sys
@@ -207,8 +208,8 @@ if mode in ("all", "engine", "gn"):
             out["engine_fsdp_fused_nogemmgather"] = dict(res=c, checksum=cc, ag_stats=dict(CK.AG_STATS))
 
 if rank == 0:
-    os.makedirs("gpurun_out", exist_ok=True)
-    with open(f"gpurun_out/multi_{world}.json", "w") as f:
-        json.dump(out, f, indent=1)
+    if len(sys.argv) > 2:
+        with open(sys.argv[2], "w") as f:
+            json.dump(out, f, indent=1)
     print(json.dumps(out))
 dist.barrier(); dist.destroy_process_group()

@@ -1,13 +1,14 @@
-"""Every public top-level name (and public method) of the reference's modules must exist under the same import path
-(`fms_fsdp.*` aliases to `fms_fsdp_b200.*`).  The reference tree is read-only input at /root/reference; the test is
-skipped when it is not mounted (e.g. in CI)."""
-import ast
+"""Every public top-level name (and public method) of the original fms-fsdp's modules must exist under the same import path
+(`fms_fsdp.*` aliases to `fms_fsdp_b200.*`) and take the same parameters.  The original's names and parameter names are
+stored in tests/golden/reference/api.json (scripts/make_reference_golden.py regenerates it from a checkout)."""
 import importlib
+import json
 import os
 
 import pytest
 
-REF = "/root/reference"
+with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference", "api.json")) as _f:
+    API = json.load(_f)
 MODULES = {
     "fms_fsdp/config/training.py": "fms_fsdp.config.training",
     "fms_fsdp/utils/config_utils.py": "fms_fsdp.utils.config_utils",
@@ -28,42 +29,33 @@ MODULES = {
 }
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not mounted")
 @pytest.mark.parametrize("path,mod", sorted(MODULES.items()))
 def test_public_names_of_reference_module_exist(path, mod):
-    tree = ast.parse(open(os.path.join(REF, path)).read())
+    ref = API[path]
     ours = importlib.import_module(mod)
-    missing = []
-    for node in tree.body:
-        if isinstance(node, (ast.FunctionDef, ast.ClassDef)) and not node.name.startswith("_"):
-            if not hasattr(ours, node.name):
-                missing.append(node.name)
-            elif isinstance(node, ast.ClassDef):
-                cls = getattr(ours, node.name)
-                missing += [f"{node.name}.{b.name}" for b in node.body
-                            if isinstance(b, ast.FunctionDef) and not b.name.startswith("_") and not hasattr(cls, b.name)]
-        elif isinstance(node, ast.Assign):
-            missing += [t.id for t in node.targets
-                        if isinstance(t, ast.Name) and not t.id.startswith("_") and not hasattr(ours, t.id)]
+    missing = [name for name in ref["functions"] if not hasattr(ours, name)]
+    for name, methods in ref["classes"].items():
+        if name.startswith("_"):
+            continue
+        if not hasattr(ours, name):
+            missing.append(name)
+            continue
+        cls = getattr(ours, name)
+        missing += [f"{name}.{m}" for m in methods if not m.startswith("_") and not hasattr(cls, m)]
+    missing += [name for name in ref["names"] if not hasattr(ours, name)]
     assert not missing, f"{mod} lacks {missing}"
 
 
-def _positional_names(fn_node):
-    a = fn_node.args
-    return [x.arg for x in a.posonlyargs + a.args if x.arg not in ("self", "cls")], [x.arg for x in a.kwonlyargs]
-
-
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not mounted")
 @pytest.mark.parametrize("path,mod", sorted(MODULES.items()))
 def test_signatures_accept_the_reference_call_forms(path, mod):
-    """Every public function / method (and ``__init__``) takes the reference's parameters under the same names and, unless it
-    takes ``*args``, at the same positions -- so both keyword and positional call sites of reference users keep working."""
+    """Every public function / method (and ``__init__``) takes the original's parameters under the same names and, unless it
+    takes ``*args``, at the same positions -- so both keyword and positional call sites of existing users keep working."""
     import inspect
-    tree = ast.parse(open(os.path.join(REF, path)).read())
+    ref = API[path]
     ours = importlib.import_module(mod)
     problems = []
 
-    def check(node, obj, label):
+    def check(sig, obj, label):
         try:
             params = list(inspect.signature(obj).parameters.values())
         except (TypeError, ValueError):
@@ -71,21 +63,21 @@ def test_signatures_accept_the_reference_call_forms(path, mod):
         names = [p.name for p in params if p.name not in ("self", "cls")]
         var_kw = any(p.kind == p.VAR_KEYWORD for p in params)
         var_pos = any(p.kind == p.VAR_POSITIONAL for p in params)
-        pos, kwonly = _positional_names(node)
-        for i, n in enumerate(pos):
+        for i, n in enumerate(sig["pos"]):
             if n not in names:
                 if not var_kw:
                     problems.append(f"{label}: no parameter {n}")
             elif names.index(n) != i and not var_pos:
                 problems.append(f"{label}: {n} is parameter {names.index(n)}, reference has it at {i}")
-        problems.extend(f"{label}: no keyword {n}" for n in kwonly if n not in names and not var_kw)
+        problems.extend(f"{label}: no keyword {n}" for n in sig["kwonly"] if n not in names and not var_kw)
 
-    for node in tree.body:
-        if isinstance(node, ast.FunctionDef) and not node.name.startswith("_") and hasattr(ours, node.name):
-            check(node, getattr(ours, node.name), node.name)
-        elif isinstance(node, ast.ClassDef) and hasattr(ours, node.name):
-            cls = getattr(ours, node.name)
-            for b in node.body:
-                if isinstance(b, ast.FunctionDef) and (b.name == "__init__" or not b.name.startswith("_")) and hasattr(cls, b.name):
-                    check(b, getattr(cls, b.name), f"{node.name}.{b.name}")
+    for name, sig in ref["functions"].items():
+        if hasattr(ours, name):
+            check(sig, getattr(ours, name), name)
+    for name, methods in ref["classes"].items():
+        if hasattr(ours, name):
+            cls = getattr(ours, name)
+            for m, sig in methods.items():
+                if hasattr(cls, m):
+                    check(sig, getattr(cls, m), f"{name}.{m}")
     assert not problems, f"{mod}: {problems}"

@@ -1,7 +1,10 @@
 """Dataset-stack properties (same catalogue the reference pins, SURVEY.md §4.1; assertions re-written).
 "Multi-node" is simulated in one process: N dataset objects with different (rank, worldsize)."""
 import copy
+import hashlib
+import json
 import os
+import tarfile
 import tempfile
 
 import pyarrow as pa
@@ -23,8 +26,7 @@ def _write(path, docs):
             w.write(pa.record_batch([d], schema=SCHEMA))
 
 
-@pytest.fixture(scope="module")
-def corpus():
+def make_corpus():
     """dataset_1: 100 docs x 100 tokens (doc i = range(100i, 100i+100)); dataset_2: 2 files x 50 docs x 50 tokens
     (one in a sub-folder); meta/combined_counts.csv.  Token values identify (doc, position)."""
     tmp = tempfile.mkdtemp()
@@ -36,6 +38,11 @@ def corpus():
         f.write("dataset/filename,documents,tokens\n/dataset_1/fullshard.arrow,100,10000\n"
                 "/dataset_2/quartershard_1.arrow,50,2500\n/dataset_2/subfolder/quartershard_2.arrow,50,2500\n")
     return tmp
+
+
+@pytest.fixture(scope="module")
+def corpus():
+    return make_corpus()
 
 
 def doc_reader(corpus, rank=0, world=1, ds="dataset_1", chunk=1000, **kw):
@@ -284,21 +291,24 @@ def test_dummy_loader_and_causal_lm():
     assert parse_data_args("a,b", "1,2.5") == (["a", "b"], [1.0, 2.5])
 
 
-# ------------------------------------------------------------------- interchange with the unmodified reference
-_REF = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "baseline", "_ref")
+# ------------------------------------------------------------------- interchange with the original fms-fsdp
+# What the original's dataset_utils produced on this corpus, and the loader checkpoint it wrote, stored under
+# tests/golden/reference (scripts/make_reference_golden.py regenerates them from a checkout of the original).
+_GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference")
 
 
-def _reference_dataset_module():
-    """The reference's own ``fms_fsdp.utils.dataset_utils`` from the offline install under baseline/_ref (DESIGN.md §4),
-    loaded under a private name so it cannot shadow this repo's ``fms_fsdp`` alias package."""
-    import importlib.util
-    path = os.path.join(_REF, "fms_fsdp", "utils", "dataset_utils.py")
-    if not os.path.exists(path):
-        pytest.skip("reference install (baseline/_ref) not present")
-    spec = importlib.util.spec_from_file_location("_reference_dataset_utils", path)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    return mod
+def _golden(key):
+    with open(os.path.join(_GOLDEN, "datasets.json")) as f:
+        return json.load(f)[key]
+
+
+@pytest.fixture(scope="module")
+def reference_checkpoints(tmp_path_factory):
+    """Loader checkpoints written by the original, one directory each."""
+    out = tmp_path_factory.mktemp("reference_checkpoints")
+    with tarfile.open(os.path.join(_GOLDEN, "loader_checkpoints.tar.xz")) as tar:
+        tar.extractall(out, filter="data")
+    return out
 
 
 def _full_stack(D, corpus, rank, world, seq=33):
@@ -309,39 +319,74 @@ def _full_stack(D, corpus, rank, world, seq=33):
     return D.PreloadBufferDataset(d, 50)
 
 
-def test_token_stream_and_loader_checkpoints_interchange_with_the_reference(corpus, tmp_path):
-    """Same corpus, same pipeline, both implementations: (1) the token streams are identical line by line; (2) a loader
-    checkpoint written by this repo is resumed by the reference's classes, and one written by the reference is resumed here
-    -- also across a change of world size (2 -> 4 ranks) -- and both continuations agree."""
+def _line_digests(it, n):
+    """A 64-bit digest of each of the next ``n`` lines: equal lines, equal digests, at a fraction of the stored size."""
+    return [hashlib.sha256(repr([int(x) for x in next(it)]).encode()).hexdigest()[:16] for _ in range(n)]
+
+
+def _state_digest(obj):
+    """Digest of a loader state (nested dicts, lists, scalars and tensors), independent of how it was pickled."""
+    h = hashlib.sha256()
+
+    def walk(o):
+        if isinstance(o, dict):
+            h.update(b"{")
+            for k in sorted(o, key=repr):
+                h.update(repr(k).encode())
+                walk(o[k])
+            h.update(b"}")
+        elif isinstance(o, (list, tuple)):
+            h.update(b"[")
+            for x in o:
+                walk(x)
+            h.update(b"]")
+        elif isinstance(o, torch.Tensor):
+            h.update(f"{o.dtype}{tuple(o.shape)}".encode() + o.contiguous().numpy().tobytes())
+        else:
+            h.update(repr(o).encode())
+    walk(obj)
+    return h.hexdigest()
+
+
+def _checkpoint_digests(path):
+    return {f: _state_digest(torch.load(os.path.join(path, f), weights_only=False)) for f in sorted(os.listdir(path))}
+
+
+def _write_checkpoint(D, corpus, path):
+    """Two ranks of the full stack each take 40 lines, then save their loader states to ``path``."""
+    stacks = [_full_stack(D, corpus, r, 2) for r in range(2)]
+    its = [iter(s) for s in stacks]
+    for it in its:
+        take(it, 40)
+    for s in stacks:
+        s.save_to_path(path)
+
+
+def _resume(D, corpus, world, path):
+    """Line digests of the next 60 lines of each of ``world`` ranks resumed from the checkpoint at ``path``."""
+    stacks = [_full_stack(D, corpus, r, world) for r in range(world)]
+    for s in stacks:
+        s.load_from_path(path)
+    return [_line_digests(iter(s), 60) for s in stacks]
+
+
+def test_token_stream_and_loader_checkpoints_interchange_with_the_reference(corpus, tmp_path, reference_checkpoints):
+    """Same corpus, same pipeline as the original fms-fsdp: (1) the token streams are identical line by line; (2) a loader
+    checkpoint written here is the one the original resumed at world 2, and resuming it here continues as the original
+    did; one written by the original resumes here at world 4 -- a change of world size -- as it does in the original."""
     import fms_fsdp_b200.utils.dataset_utils as OURS
-    REF = _reference_dataset_module()
+    assert _line_digests(iter(_full_stack(OURS, corpus, 0, 1)), 300) == _golden("stream")
 
-    a, b = iter(_full_stack(OURS, corpus, 0, 1)), iter(_full_stack(REF, corpus, 0, 1))
-    for _ in range(300):
-        assert list(next(a)) == list(next(b))
+    ck = str(tmp_path / "ours_to_ref")
+    _write_checkpoint(OURS, corpus, ck)
+    assert _checkpoint_digests(ck) == _golden("ours_to_ref checkpoint")
+    assert _resume(OURS, corpus, 2, ck) == _golden("ours_to_ref")
 
-    # (2a) ours writes at world 2, the reference resumes at world 2; (2b) the reference writes, we resume at world 4
-    for writer, reader, new_world, tag in ((OURS, REF, 2, "ours_to_ref"), (REF, OURS, 4, "ref_to_ours")):
-        ck = str(tmp_path / tag)
-        stacks = [_full_stack(writer, corpus, r, 2) for r in range(2)]
-        its = [iter(s) for s in stacks]
-        for it in its:
-            take(it, 40)
-        for s in stacks:
-            s.save_to_path(ck)
-        resumed_other = [_full_stack(reader, corpus, r, new_world) for r in range(new_world)]
-        resumed_same = [_full_stack(writer, corpus, r, new_world) for r in range(new_world)]
-        for s in resumed_other + resumed_same:
-            s.load_from_path(ck)
-        for x, y in zip(resumed_other, resumed_same):
-            ix, iy = iter(x), iter(y)
-            for _ in range(60):
-                assert list(next(ix)) == list(next(iy)), tag
+    assert _resume(OURS, corpus, 4, str(reference_checkpoints / "ref_to_ours")) == _golden("ref_to_ours")
 
 
 # ------------------------------------------------------------------------ parquet / auto handlers (raw text + tokenizer)
-@pytest.fixture(scope="module")
-def text_corpus():
+def make_text_corpus():
     """A local word-level tokenizer (saved so ``AutoTokenizer.from_pretrained(dir)`` works offline; it adds <s> ... </s> like
     the HF Llama tokenizers do) and a corpus with one parquet text shard and one pre-tokenised arrow shard."""
     import pyarrow.parquet as pq
@@ -359,6 +404,16 @@ def text_corpus():
     pq.write_table(pa.table({"text": docs, "other": list(range(40))}), f"{tmp}/data/mix/part_0.parquet")
     _write(f"{tmp}/data/mix/part_1.arrow", [[300 + 50 * d + j for j in range(30)] for d in range(20)])
     return tmp, docs, vocab
+
+
+@pytest.fixture(scope="module")
+def text_corpus():
+    return make_text_corpus()
+
+
+def _text_reader(D, tmp):
+    return D.StreamingDocDataset(f"{tmp}/data/mix", 0, 1, D.AutoHandler(f"{tmp}/tok", "text"), 0, strip_tokens={1, 2}, seed=3,
+                                 max_chunksize=16)
 
 
 def test_parquet_and_auto_handlers_tokenise_strip_and_match_the_reference(text_corpus):
@@ -380,15 +435,9 @@ def test_parquet_and_auto_handlers_tokenise_strip_and_match_the_reference(text_c
     r = a.open(path)
     assert a.get(r, 0, {1, 2}) == [vocab[w] for w in docs[0].split()]
 
-    # the whole reader on the mixed folder: same documents, same order as the unmodified reference classes
-    REF = _reference_dataset_module()
-    ours = StreamingDocDataset(f"{tmp}/data/mix", 0, 1, AutoHandler(f"{tmp}/tok", "text"), 0, strip_tokens={1, 2}, seed=3,
-                               max_chunksize=16)
-    theirs = REF.StreamingDocDataset(f"{tmp}/data/mix", 0, 1, REF.AutoHandler(f"{tmp}/tok", "text"), 0, strip_tokens={1, 2},
-                                     seed=3, max_chunksize=16)
-    io, it = iter(ours), iter(theirs)
-    for _ in range(200):
-        assert list(next(io)) == list(next(it))
+    # the whole reader on the mixed folder: same documents, same order as the original's classes
+    import fms_fsdp_b200.utils.dataset_utils as OURS
+    assert _line_digests(iter(_text_reader(OURS, tmp)), 200) == _golden("text_reader")
 
 
 def test_get_data_loader_with_file_type_auto_runs_on_text_and_token_shards(text_corpus, tmp_path):
@@ -411,98 +460,118 @@ def test_get_data_loader_with_file_type_auto_runs_on_text_and_token_shards(text_
     assert any(10 <= t < 210 for t in seen) and any(t >= 300 for t in seen)   # both the text and the token shard are read
 
 
-@pytest.mark.parametrize("kw", [dict(pack_hard=False, pad_token=-5), dict(pack_hard=False, pad_token=-5, bos_token=-2, eos_token=-3),
-                                dict(pack_hard=True, bos_token=-2), dict(pack_hard=True, eos_token=-3, bos_token=-2)])
+PACKER_KW = [dict(pack_hard=False, pad_token=-5), dict(pack_hard=False, pad_token=-5, bos_token=-2, eos_token=-3),
+             dict(pack_hard=True, bos_token=-2), dict(pack_hard=True, eos_token=-3, bos_token=-2)]
+
+
+def _packer_stack(D, corpus, kw):
+    d = D.StreamingDocDataset(corpus, 0, 1, D.ArrowHandler(), -1, seed=11, max_chunksize=40)
+    d = D.SamplingDataset(corpus, d, -1, datasets=["dataset_1", "dataset_2"], weights=[1, 2], verbose=False)
+    return D.BufferDataset(d, 37, **kw)
+
+
+@pytest.mark.parametrize("kw", PACKER_KW)
 def test_line_packer_modes_equal_the_reference(corpus, kw):
-    """Every packing mode of ``BufferDataset`` (hard / soft packing, per-line BOS / EOS, padding) against the unmodified
-    reference class on the same sampled two-dataset stream."""
+    """Every packing mode of ``BufferDataset`` (hard / soft packing, per-line BOS / EOS, padding) against the original
+    class on the same sampled two-dataset stream."""
     import fms_fsdp_b200.utils.dataset_utils as OURS
-    REF = _reference_dataset_module()
-
-    def build(D):
-        d = D.StreamingDocDataset(corpus, 0, 1, D.ArrowHandler(), -1, seed=11, max_chunksize=40)
-        d = D.SamplingDataset(corpus, d, -1, datasets=["dataset_1", "dataset_2"], weights=[1, 2], verbose=False)
-        return D.BufferDataset(d, 37, **kw)
-
-    a, b = iter(build(OURS)), iter(build(REF))
-    for _ in range(250):
-        assert list(next(a)) == list(next(b))
+    assert _line_digests(iter(_packer_stack(OURS, corpus, kw)), 250) == _golden(f"packer {kw!r}")
 
 
-@pytest.mark.parametrize("world,rank,bos,min_len,nlog", [(3, 1, None, 1, 6), (2, 0, -9, 3, 8), (4, 3, -9, 60, 12), (1, 0, None, 101, 5)])
+PARTITION_CASES = [(3, 1, None, 1, 6), (2, 0, -9, 3, 8), (4, 3, -9, 60, 12), (1, 0, None, 101, 5)]
+
+
+def _partition_stack(D, corpus, world, rank, bos, min_len, nlog):
+    d = D.StreamingDocDataset(os.path.join(corpus, "dataset_2") if min_len < 101 else corpus, rank, world, D.ArrowHandler(),
+                              -1, bos_token=bos, min_length=min_len, seed=5, max_chunksize=33)
+    return D.ScalableShardDataset(d, -1, n_logical_shards=nlog * world)
+
+
+@pytest.mark.parametrize("world,rank,bos,min_len,nlog", PARTITION_CASES)
 def test_reader_partitioning_options_equal_the_reference(corpus, world, rank, bos, min_len, nlog):
     """Document reader + logical shards under different partitionings, BOS insertion and minimum document lengths (which
-    drop all of dataset_2's 50-token documents at 60 and everything at 101): chunk for chunk what the reference yields."""
+    drop all of dataset_2's 50-token documents at 60 and everything at 101): chunk for chunk what the original yields."""
     # (50 tokens + delimiter + BOS = 52 < 60)
     import fms_fsdp_b200.utils.dataset_utils as OURS
-    REF = _reference_dataset_module()
-
-    def build(D):
-        d = D.StreamingDocDataset(os.path.join(corpus, "dataset_2") if min_len < 101 else corpus, rank, world, D.ArrowHandler(),
-                                  -1, bos_token=bos, min_length=min_len, seed=5, max_chunksize=33)
-        return D.ScalableShardDataset(d, -1, n_logical_shards=nlog * world)
-
+    case = (world, rank, bos, min_len, nlog)
     if min_len >= 60:
-        # nothing survives the length filter: the reference spins forever in that case; here it is an error that says why
+        # nothing survives the length filter: the original spins forever in that case; here it is an error that says why
         with pytest.raises(RuntimeError, match="min_length"):
-            next(iter(build(OURS)))
+            next(iter(_partition_stack(OURS, corpus, *case)))
         return
-    a, b = iter(build(OURS)), iter(build(REF))
-    for _ in range(150):
-        assert list(next(a)) == list(next(b))
+    assert _line_digests(iter(_partition_stack(OURS, corpus, *case)), 150) == _golden(f"partition {case!r}")
 
 
-@pytest.mark.parametrize("writer_is_ours,old_world,new_world", [(True, 3, 2), (False, 4, 6), (True, 6, 4), (False, 2, 1)])
-def test_rescaled_resume_equals_the_reference_for_more_world_size_pairs(corpus, tmp_path, writer_is_ours, old_world, new_world):
-    """Loader checkpoints written at ``old_world`` ranks by one implementation, resumed at ``new_world`` ranks by both: every
-    new rank continues with the same lines in either implementation (shrinking, growing, non-divisible pairs)."""
-    import fms_fsdp_b200.utils.dataset_utils as OURS
-    REF = _reference_dataset_module()
-    writer = OURS if writer_is_ours else REF
-    ck = str(tmp_path / "ck")
+RESCALE_CASES = [(True, 3, 2), (False, 4, 6), (True, 6, 4), (False, 2, 1)]
 
-    def stack(D, rank, world):
-        d = D.StreamingDocDataset(corpus, rank, world, D.ArrowHandler(), -1, strip_tokens={-1}, min_length=3, seed=7)
-        d = D.ScalableShardDataset(d, -1, n_logical_shards=12)
-        d = D.SamplingDataset(corpus, d, -1, datasets=["dataset_1", "dataset_2"], weights=[3, 1], verbose=False)
-        d = D.BufferDataset(d, 33, bos_token=None, eos_token=None, pack_hard=True)
-        return D.PreloadBufferDataset(d, 50)
 
-    olds = [stack(writer, r, old_world) for r in range(old_world)]
+def _rescale_stack(D, corpus, rank, world):
+    d = D.StreamingDocDataset(corpus, rank, world, D.ArrowHandler(), -1, strip_tokens={-1}, min_length=3, seed=7)
+    d = D.ScalableShardDataset(d, -1, n_logical_shards=12)
+    d = D.SamplingDataset(corpus, d, -1, datasets=["dataset_1", "dataset_2"], weights=[3, 1], verbose=False)
+    d = D.BufferDataset(d, 33, bos_token=None, eos_token=None, pack_hard=True)
+    return D.PreloadBufferDataset(d, 50)
+
+
+def _rescale_write(D, corpus, world, path):
+    olds = [_rescale_stack(D, corpus, r, world) for r in range(world)]
     for s in olds:
         take(iter(s), 30)
     for s in olds:
-        s.save_to_path(ck)
-    for r in range(new_world):
-        a, b = stack(OURS, r, new_world), stack(REF, r, new_world)
-        a.load_from_path(ck); b.load_from_path(ck)
-        ia, ib = iter(a), iter(b)
-        for _ in range(40):
-            assert list(next(ia)) == list(next(ib)), (r, new_world)
+        s.save_to_path(path)
+
+
+def _rescale_resume(D, corpus, world, path):
+    out = []
+    for r in range(world):
+        s = _rescale_stack(D, corpus, r, world)
+        s.load_from_path(path)
+        out.append(_line_digests(iter(s), 40))
+    return out
+
+
+@pytest.mark.parametrize("writer_is_ours,old_world,new_world", RESCALE_CASES)
+def test_rescaled_resume_equals_the_reference_for_more_world_size_pairs(corpus, tmp_path, reference_checkpoints, writer_is_ours,
+                                                                        old_world, new_world):
+    """Loader checkpoints written at ``old_world`` ranks by one implementation, resumed at ``new_world`` ranks by both: every
+    new rank continues with the same lines in either implementation (shrinking, growing, non-divisible pairs).  A checkpoint
+    written here must be the one the original resumed; one written by the original is stored."""
+    import fms_fsdp_b200.utils.dataset_utils as OURS
+    key = f"rescale {(writer_is_ours, old_world, new_world)!r}"
+    if writer_is_ours:
+        ck = str(tmp_path / "ck")
+        _rescale_write(OURS, corpus, old_world, ck)
+        assert _checkpoint_digests(ck) == _golden(key + " checkpoint")
+    else:
+        ck = str(reference_checkpoints / f"rescale_{old_world}_to_{new_world}")
+    assert _rescale_resume(OURS, corpus, new_world, ck) == _golden(key)
+
+
+def _worker_loader(D, corpus, path):
+    d = D.StreamingDocDataset(corpus, 1, 2, D.ArrowHandler(), -1, min_length=3, seed=3)
+    d = D.ScalableShardDataset(d, -1, n_logical_shards=8)
+    d = D.SamplingDataset(corpus, d, -1, datasets=["dataset_1", "dataset_2"], weights=[1, 1], verbose=False)
+    d = D.BufferDataset(d, 21, pack_hard=True)
+    d = D.PreloadBufferDataset(d, 20)
+    d = D.PreprocessDataset(d, torch.IntTensor)
+    d = D.CheckpointDataset(d, path, 5, 2, path)
+    return torch.utils.data.DataLoader(d, num_workers=2, batch_size=2)
+
+
+def _worker_run(D, corpus, path):
+    """Digests of 24 batches through two worker processes, and the auto-checkpoints they left under ``path``."""
+    it = iter(_worker_loader(D, corpus, path))
+    batches = [_state_digest(next(it))[:16] for _ in range(24)]
+    del it
+    steps = sorted(os.listdir(os.path.join(path, "checkpoints")))
+    return {"batches": batches, "checkpoints": steps,
+            "last_checkpoint_files": sorted(os.listdir(os.path.join(path, "checkpoints", steps[-1]))) if steps else []}
 
 
 def test_multi_worker_dataloader_stream_equals_the_reference(corpus, tmp_path):
     """Through ``torch.utils.data.DataLoader(num_workers=2)``: each worker process derives its own partition from
-    (rank, world, worker id); the batches of both implementations are identical, including the in-worker auto-checkpoints."""
+    (rank, world, worker id); the batches are the original's, and so are the in-worker auto-checkpoints."""
     import fms_fsdp_b200.utils.dataset_utils as OURS
-    REF = _reference_dataset_module()
-
-    def loader(D, tag):
-        d = D.StreamingDocDataset(corpus, 1, 2, D.ArrowHandler(), -1, min_length=3, seed=3)
-        d = D.ScalableShardDataset(d, -1, n_logical_shards=8)
-        d = D.SamplingDataset(corpus, d, -1, datasets=["dataset_1", "dataset_2"], weights=[1, 1], verbose=False)
-        d = D.BufferDataset(d, 21, pack_hard=True)
-        d = D.PreloadBufferDataset(d, 20)
-        d = D.PreprocessDataset(d, torch.IntTensor)
-        d = D.CheckpointDataset(d, str(tmp_path / tag), 5, 2, str(tmp_path / tag))
-        return torch.utils.data.DataLoader(d, num_workers=2, batch_size=2)
-
-    a, b = iter(loader(OURS, "ours")), iter(loader(REF, "ref"))
-    for _ in range(24):
-        assert torch.equal(next(a), next(b))
-    del a, b
-    mine = sorted(os.listdir(tmp_path / "ours" / "checkpoints"))
-    theirs = sorted(os.listdir(tmp_path / "ref" / "checkpoints"))
-    assert mine == theirs and mine, (mine, theirs)
-    step_dir = mine[-1]
-    assert sorted(os.listdir(tmp_path / "ours" / "checkpoints" / step_dir)) == sorted(os.listdir(tmp_path / "ref" / "checkpoints" / step_dir))
+    mine = _worker_run(OURS, corpus, str(tmp_path / "ours"))
+    assert mine["checkpoints"], mine
+    assert mine == _golden("multi_worker")

@@ -188,21 +188,21 @@ def test_smoke_entry():
     g.smoke()
 
 
-if torch.cuda.device_count() >= 2:
-    # Real NVLink run (2 ranks).  On the 1-GPU test box the same kernels are exercised through local pointer tables in
-    # tests/test_gpu_collectives_1gpu.py, so this test only EXISTS where it can run (nothing is skipped on 1 GPU).
-    def test_fused_collectives_two_gpus():
-        env = dict(os.environ, PYTHONPATH=ROOT)
-        r = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2",
-                            "--master-addr", "127.0.0.1", "--master-port", "29541",
-                            os.path.join(ROOT, "scripts", "gpu_multi_check.py"), "all"],
-                           env=env, capture_output=True, text=True, timeout=600, cwd=ROOT)
-        assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
-        import json
-        out = json.load(open(os.path.join(ROOT, "gpurun_out", "multi_2.json")))
-        assert out["allgather_equal"] and out["reduce_scatter_maxdiff"] < 1e-3
-        f, t = out["engine_fsdp"]["fused"], out["engine_fsdp"]["torch"]
-        assert all(abs(a[1] - b[1]) < 2e-2 * b[1] for a, b in zip(f, t))
+# Real NVLink run (2 ranks).  On one GPU the same kernels are exercised through local pointer tables in
+# tests/test_gpu_collectives_1gpu.py.
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs")
+def test_fused_collectives_two_gpus(tmp_path):
+    env = dict(os.environ, PYTHONPATH=ROOT)
+    r = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2",
+                        "--master-addr", "127.0.0.1", "--master-port", "29541",
+                        os.path.join(ROOT, "scripts", "gpu_multi_check.py"), "all", str(tmp_path / "multi_2.json")],
+                       env=env, capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
+    import json
+    out = json.load(open(tmp_path / "multi_2.json"))
+    assert out["allgather_equal"] and out["reduce_scatter_maxdiff"] < 1e-3
+    f, t = out["engine_fsdp"]["fused"], out["engine_fsdp"]["torch"]
+    assert all(abs(a[1] - b[1]) < 2e-2 * b[1] for a, b in zip(f, t))
 
 
 @pytest.mark.parametrize("shape", [(2, 256, 8, 64, 1, 128), (1, 384, 8, 64, 2, 64)])
