@@ -73,6 +73,11 @@ def main():
             print(json.dumps({"impl": "reference", "unavailable": why[:300]}))
         return
 
+    if a.model.startswith("qwen"):
+        if rank == 0:
+            print(json.dumps({"impl": "reference", "unavailable": "the reference model zoo has no Qwen2 (q/k/v-bias) variant"}))
+        return
+
     cfg = config.train_config()
     update_config(cfg, model_variant=a.model, use_dummy_dataset=True, sharding_strategy="fsdp", seq_length=a.seq,
                   batch_size=a.batch, low_cpu_fsdp=True, use_torch_compile=not a.no_compile,

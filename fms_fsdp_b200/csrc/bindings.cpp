@@ -68,6 +68,8 @@ DECL int b200_attn_bwd(const void*, const void*, const void*, const float*, void
 DECL void b200_gemm2_set_rope(const float*, int, int, int);
 DECL void b200_gemm2_set_swiglu(void*, int, int, int);
 DECL int b200_gemm2_fp8(const void*, const void*, void*, const float*, const float*, int, int, int, int, int, int, cudaStream_t);
+DECL int b200_bias_grad_partials(int, int);
+DECL int b200_bias_grad(const void*, float*, void*, int, int, int, int, cudaStream_t);
 DECL int b200_quant_rowwise_e4m3(const void*, void*, float*, int, int, int, int, cudaStream_t);
 DECL void b200_gemm2_set_push(void* const*, long long, long long, int, int, int);
 DECL int b200_p2p_push_range(const void*, void* const*, long long, long long, long long, int, cudaStream_t);
@@ -105,9 +107,20 @@ inline void need_rowmajor2d(const at::Tensor& t, const char* name) {
               name, " must be 16-byte aligned (ptr and row stride)");
 }
 
+// epilogue flag (csrc/gemm2_sm100.cu P_EPI_BIAS): + bias[col] before the store / RoPE; the bias travels in the R slot
+constexpr int kEpiBias = 16;
+// bias [N] bf16, contiguous, 16-byte aligned: returns its pointer (the R operand of the launch)
+inline const void* bias_operand(const c10::optional<at::Tensor>& bias, int64_t N) {
+  need(*bias, "bias", at::kBFloat16);
+  TORCH_CHECK(bias->is_contiguous() && bias->numel() == N && (reinterpret_cast<uintptr_t>(bias->data_ptr()) & 15) == 0,
+              "bias must be a contiguous, 16-byte aligned [N] tensor");
+  return bias->data_ptr();
+}
+
 // layout: 0 = nt, 1 = nn, 2 = tn ; epi: 0 store, 1 +residual, 2 accumulate into c
+// bias (nt, epi 0 / 3, CTA-pair kernel, bf16 output): c = a b^T + bias[col] (then RoPE for epi 3)
 void gemm(const at::Tensor& a, const at::Tensor& b, at::Tensor& c, int64_t layout, int64_t epi,
-          const c10::optional<at::Tensor>& residual) {
+          const c10::optional<at::Tensor>& residual, const c10::optional<at::Tensor>& bias) {
   c10::cuda::CUDAGuard guard(a.device());
   need(a, "a", at::kBFloat16);
   need(b, "b", at::kBFloat16);
@@ -142,6 +155,13 @@ void gemm(const at::Tensor& a, const at::Tensor& b, at::Tensor& c, int64_t layou
   TORCH_CHECK(epi != 3 || (g_gemm_2cta && M >= 256 && layout == 0 && c.scalar_type() == at::kBFloat16),
               "RoPE epilogue: CTA-pair kernel, nt layout, bf16 output only (call set_gemm_rope first)");
   TORCH_CHECK(epi != 4, "push epilogue: use gemm_push (no output tensor)");
+  if (bias.has_value() && bias->defined()) {
+    TORCH_CHECK((epi == 0 || epi == 3) && layout == 0 && g_gemm_2cta && M >= 256 && c.scalar_type() == at::kBFloat16,
+                "bias epilogue: CTA-pair kernel, nt layout, store or RoPE epilogue, bf16 output only");
+    r = bias_operand(bias, N);
+    ldr = 0;
+    epi |= kEpiBias;
+  }
   // CTA-pair kernel (cta_group::2, 256x256 tiles) for anything with at least one full pair tile of rows
   if (g_gemm_2cta && M >= 256) {
     check(b200_gemm2_bf16(a.data_ptr(), b.data_ptr(), c.data_ptr(), r, M, N, K, a.stride(0), b.stride(0), c.stride(0),
@@ -454,7 +474,7 @@ bool get_gemm_2cta() { return g_gemm_2cta; }
 void gemm_ag(const at::Tensor& a, const at::Tensor& b, const c10::optional<at::Tensor>& c_opt, int64_t layout, int64_t epi,
              const c10::optional<at::Tensor>& residual, const at::Tensor& peer_ptrs, at::Tensor& full,
              int64_t shard_bytes, int64_t begin, int64_t end, int64_t world, int64_t rank, at::Tensor& flags,
-             int64_t epoch, bool dependent) {
+             int64_t epoch, bool dependent, const c10::optional<at::Tensor>& bias) {
   c10::cuda::CUDAGuard guard(a.device());
   need(a, "a", at::kBFloat16);
   need(b, "b", at::kBFloat16);
@@ -488,6 +508,12 @@ void gemm_ag(const at::Tensor& a, const at::Tensor& b, const c10::optional<at::T
     need(*residual, "residual", at::kBFloat16);
     r = residual->data_ptr();
     ldr = residual->stride(0);
+  }
+  if (bias.has_value() && bias->defined()) {
+    TORCH_CHECK((epi == 0 || epi == 3) && layout == 0, "bias epilogue: nt layout, store or RoPE epilogue");
+    r = bias_operand(bias, N);
+    ldr = 0;
+    epi |= kEpiBias;
   }
   check(b200_gemm2_ag_bf16(a.data_ptr(), b.data_ptr(), c.data_ptr(), r, M, N, K, a.stride(0), b.stride(0), c.stride(0), ldr,
                            a_mn, b_mn, (int)epi, (const void* const*)peer_ptrs.data_ptr(), full.data_ptr(),
@@ -530,6 +556,19 @@ void gemm_fp8(const at::Tensor& aq, const at::Tensor& bq, const at::Tensor& sa, 
               sa.is_contiguous() && sb.is_contiguous(), "gemm_fp8: shape mismatch");
   check(b200_gemm2_fp8(aq.data_ptr(), bq.data_ptr(), c.data_ptr(), sa.data_ptr<float>(), sb.data_ptr<float>(), M, N, K,
                        (int)aq.stride(0), (int)bq.stride(0), (int)c.stride(0), cur_stream()), "gemm2_fp8_tcgen05");
+}
+// db [N] (bf16 or fp32) = column sums of dy [M, N] bf16, or db += them (accumulate); deterministic (fixed split, no atomics)
+void bias_grad(const at::Tensor& dy, at::Tensor& db, bool accumulate) {
+  c10::cuda::CUDAGuard guard(dy.device());
+  need(dy, "dy", at::kBFloat16);
+  need_rowmajor2d(dy, "dy");
+  const int M = dy.size(0), N = dy.size(1);
+  TORCH_CHECK(dy.is_contiguous() && N % 8 == 0, "bias_grad: dy must be contiguous [M, N] with N % 8 == 0");
+  TORCH_CHECK(db.is_cuda() && db.is_contiguous() && db.numel() == N &&
+              (db.scalar_type() == at::kBFloat16 || db.scalar_type() == at::kFloat), "bias_grad: db must be [N] bf16 or fp32");
+  auto part = at::empty({b200_bias_grad_partials(M, N), N}, dy.options().dtype(at::kFloat));
+  check(b200_bias_grad(dy.data_ptr(), part.data_ptr<float>(), db.data_ptr(), db.scalar_type() == at::kFloat ? 1 : 0, M, N,
+                       accumulate ? 1 : 0, cur_stream()), "bias_grad", 2);
 }
 void p2p_gather_range(const at::Tensor& peer_ptrs, at::Tensor& full, int64_t shard_bytes, int64_t begin, int64_t end) {
   c10::cuda::CUDAGuard guard(full.device());
@@ -766,7 +805,10 @@ std::vector<at::Tensor> selective_scan_bwd(const at::Tensor& dy, const at::Tenso
 
 PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
   m.doc() = "fms_fsdp_b200 sm_100a kernels";
-  m.def("gemm", &gemm);
+  m.def("gemm", &gemm, py::arg("a"), py::arg("b"), py::arg("c"), py::arg("layout"), py::arg("epi"), py::arg("residual"),
+        py::arg("bias") = py::none());
+  m.def("bias_grad", &bias_grad, py::arg("dy"), py::arg("db"), py::arg("accumulate") = false);
+  m.def("bias_grad_partials", [](int64_t M, int64_t N) { return (int64_t)b200_bias_grad_partials((int)M, (int)N); });
   m.def("rmsnorm_fwd", &rmsnorm_fwd);
   m.def("rmsnorm_bwd", &rmsnorm_bwd, py::arg("dy"), py::arg("x"), py::arg("w"), py::arg("rstd"), py::arg("dres") = py::none());
   m.def("add_rmsnorm_fwd", &add_rmsnorm_fwd);
@@ -830,7 +872,9 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
   m.def("set_attn_bwd_version", &set_attn_bwd_version);
   m.def("set_gemm_2cta", &set_gemm_2cta);
   m.def("get_gemm_2cta", &get_gemm_2cta);
-  m.def("gemm_ag", &gemm_ag);
+  m.def("gemm_ag", &gemm_ag, py::arg("a"), py::arg("b"), py::arg("c"), py::arg("layout"), py::arg("epi"), py::arg("residual"),
+        py::arg("peer_ptrs"), py::arg("full"), py::arg("shard_bytes"), py::arg("begin"), py::arg("end"), py::arg("world"),
+        py::arg("rank"), py::arg("flags"), py::arg("epoch"), py::arg("dependent"), py::arg("bias") = py::none());
   m.def("gemm_push", &gemm_push);
   m.def("quant_rowwise_e4m3", &quant_rowwise_e4m3);
   m.def("gemm_fp8", &gemm_fp8);

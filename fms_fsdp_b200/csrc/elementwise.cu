@@ -723,6 +723,49 @@ __global__ void sumsq_kernel(const T* __restrict__ x, size_t n, float* __restric
   if (threadIdx.x == 0) atomicAdd(out, s);
 }
 
+// ------------------------------------------------------------- bias gradient: db[n] = sum_m dy[m, n]
+// Deterministic two-pass column sum.  Pass 1: CTA (column block of 256, row slice p) -- 32 lanes x 8 columns (one
+// 16-byte load per row, a warp reads 512 contiguous bytes) x 8 warps striding the slice's rows; the warps' sums are
+// combined in a fixed order into part[p, n].  Pass 2: one thread per column adds the P partials in order p = 0..P-1.
+// The split depends on (M, N) only, so two runs give bitwise-equal results; no atomics.
+constexpr int BG_COLS = 256;
+__global__ void __launch_bounds__(256) bias_grad_partial_kernel(const __nv_bfloat16* __restrict__ dy, float* __restrict__ part,
+                                                                int M, int N, int rows_per) {
+  __shared__ float sh[8][BG_COLS + 4];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const int c = blockIdx.x * BG_COLS + lane * 8;
+  const int r0 = blockIdx.y * rows_per, r1 = min(M, r0 + rows_per);
+  float s[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+  if (c < N) {
+#pragma unroll 4
+    for (int r = r0 + w; r < r1; r += 8) {
+      const uint4 v = *reinterpret_cast<const uint4*>(dy + (size_t)r * N + c);
+      const float2 a = unpack_bf16x2(v.x), b = unpack_bf16x2(v.y), e = unpack_bf16x2(v.z), f = unpack_bf16x2(v.w);
+      s[0] += a.x; s[1] += a.y; s[2] += b.x; s[3] += b.y; s[4] += e.x; s[5] += e.y; s[6] += f.x; s[7] += f.y;
+    }
+  }
+#pragma unroll
+  for (int i = 0; i < 8; ++i) sh[w][lane * 8 + i] = s[i];
+  __syncthreads();
+  const int col = blockIdx.x * BG_COLS + threadIdx.x;
+  if (col < N) {
+    float t = 0.f;
+#pragma unroll
+    for (int k = 0; k < 8; ++k) t += sh[k][threadIdx.x];
+    part[(size_t)blockIdx.y * N + col] = t;
+  }
+}
+template <typename OutT>
+__global__ void __launch_bounds__(256) bias_grad_final_kernel(const float* __restrict__ part, OutT* __restrict__ out, int P,
+                                                              int N, int accumulate) {
+  const int col = blockIdx.x * blockDim.x + threadIdx.x;
+  if (col >= N) return;
+  float t = 0.f;
+  for (int p = 0; p < P; ++p) t += part[(size_t)p * N + col];
+  if (accumulate) t += static_cast<float>(out[col]);
+  out[col] = static_cast<OutT>(t);
+}
+
 static inline int grid_for(size_t work_items, int threads, int max_blocks = 148 * 8) {
   size_t b = (work_items + threads - 1) / threads;
   if (b < 1) b = 1;
@@ -933,5 +976,30 @@ extern "C" int b200_quant_rowwise_e4m3(const void* x, void* q, float* scale, int
   const int warps = 8;
   b200::quant_rowwise_e4m3_kernel<<<(rows + warps - 1) / warps, warps * 32, 0, s>>>((const __nv_bfloat16*)x, (uint8_t*)q, scale,
                                                                                    rows, K, ldx, ldq);
+  return (int)cudaGetLastError();
+}
+
+// db[N] (bf16 or fp32; written, or added to when accumulate) = column sums of dy [M, N] bf16 (row pitch N).
+// part: fp32 workspace of b200_bias_grad_partials(M, N) x N elements.
+extern "C" int b200_bias_grad_partials(int M, int N) {
+  const int col_blocks = (N + b200::BG_COLS - 1) / b200::BG_COLS;
+  int P = (148 * 4 + col_blocks - 1) / col_blocks;     // about four CTAs per SM in pass 1
+  const int max_p = (M + 63) / 64;                     // at least 64 rows per slice
+  if (P > max_p) P = max_p;
+  if (P < 1) P = 1;
+  const int rows_per = (M + P - 1) / P;
+  return M > 0 ? (M + rows_per - 1) / rows_per : 1;
+}
+extern "C" int b200_bias_grad(const void* dy, float* part, void* db, int db_is_f32, int M, int N, int accumulate,
+                              cudaStream_t s) {
+  if ((N % 8) || M < 0 || (reinterpret_cast<uintptr_t>(dy) & 15)) return -1;
+  const int P = b200_bias_grad_partials(M, N);
+  const int rows_per = M > 0 ? (M + P - 1) / P : 1;
+  b200::bias_grad_partial_kernel<<<dim3((N + b200::BG_COLS - 1) / b200::BG_COLS, P), 256, 0, s>>>(
+      (const __nv_bfloat16*)dy, part, M, N, rows_per);
+  if (db_is_f32)
+    b200::bias_grad_final_kernel<float><<<(N + 255) / 256, 256, 0, s>>>(part, (float*)db, P, N, accumulate);
+  else
+    b200::bias_grad_final_kernel<__nv_bfloat16><<<(N + 255) / 256, 256, 0, s>>>(part, (__nv_bfloat16*)db, P, N, accumulate);
   return (int)cudaGetLastError();
 }

@@ -32,6 +32,10 @@ constexpr int PUSH_STAGE_BYTES = 4 * 32 * PUSH_ROW_PITCH;   // 18 KiB per CTA
 
 enum { P_EPI_STORE = 0, P_EPI_RESIDUAL = 1, P_EPI_ACCUM = 2, P_EPI_ROPE = 3, P_EPI_PUSH = 4, P_EPI_SWIGLU = 5,
        P_EPI_SWIGLU_BWD = 6, P_EPI_SCALE = 7 };
+// flag OR-ed into P_EPI_STORE / P_EPI_ROPE: add the bf16 bias b[col] (16-byte aligned, [N]; passed in Gemm2Params::R)
+// to the fp32 accumulator before anything else the epilogue does (qkv = x W^T + b, then RoPE).  A flag bit of the
+// same template argument keeps the bias-free instantiations' names, parameter layout and code exactly as they were.
+constexpr int P_EPI_BIAS = 16;
 
 
 // L2-friendly rasterisation: sweep all n-tiles for a band of GROUP_M m-tiles before moving to the next band, so the
@@ -148,10 +152,13 @@ B200_DEVINL void bulk_store_s2g(void* gdst, const void* ssrc, uint32_t bytes) {
                ::"l"(gdst), "r"(smem_u32(ssrc)), "r"(bytes) : "memory");
 }
 
-template <bool A_MN, bool B_MN, int EPI, typename OutT, bool AG, bool FP8 = false>
+template <bool A_MN, bool B_MN, int EPI_BITS, typename OutT, bool AG, bool FP8 = false>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(P_THREADS + (AG ? 32 * AG_WARPS : 0), 1)
 gemm2_bf16_tcgen05(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, Gemm2Params p,
                    AgParams ag) {
+  constexpr int EPI = EPI_BITS & ~P_EPI_BIAS;
+  constexpr bool BIAS = (EPI_BITS & P_EPI_BIAS) != 0;
+  static_assert(!BIAS || ((EPI == P_EPI_STORE || EPI == P_EPI_ROPE) && sizeof(OutT) == 2), "bias: bf16 store / RoPE only");
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* bar_base = smem + P_STAGES * P_STAGE_BYTES;
@@ -415,6 +422,14 @@ gemm2_bf16_tcgen05(const __grid_constant__ CUtensorMap tmA, const __grid_constan
       } else {
 #pragma unroll 1
       for (int c = 0; c < P_BN; c += 64) {
+        uint4 bias8[BIAS ? 8 : 1];
+        if constexpr (BIAS) {   // the chunk's 64 bias values, loaded before the TMEM wait so that their latency overlaps it;
+                                // every lane of the warp reads the same bytes (broadcast)
+#pragma unroll
+          for (int g = 0; g < 8; ++g)
+            if (n0 + c + g * 8 < p.N)
+              bias8[g] = *reinterpret_cast<const uint4*>(reinterpret_cast<const __nv_bfloat16*>(p.R) + n0 + c + g * 8);
+        }
         uint32_t v0[32], v1[32];
         tmem_ld_32x32b_x32(taddr + c, v0);
         tmem_ld_32x32b_x32(taddr + c + 32, v1);
@@ -469,6 +484,12 @@ gemm2_bf16_tcgen05(const __grid_constant__ CUtensorMap tmA, const __grid_constan
                 float f[8];
 #pragma unroll
                 for (int i = 0; i < 8; ++i) f[i] = __uint_as_float(v[g * 8 + i]);
+                if constexpr (BIAS) {
+                  const uint4 bv = bias8[h * 4 + g];
+                  const float2 b0 = unpack_bf16x2(bv.x), b1 = unpack_bf16x2(bv.y), b2 = unpack_bf16x2(bv.z),
+                               b3 = unpack_bf16x2(bv.w);
+                  f[0] += b0.x; f[1] += b0.y; f[2] += b1.x; f[3] += b1.y; f[4] += b2.x; f[5] += b2.y; f[6] += b3.x; f[7] += b3.y;
+                }
                 if constexpr (EPI == P_EPI_PUSH) {
                   const long long e = p.push_off + (long long)row * p.ldc + (cb + g * 8);
                   const long long owner = e / p.push_n;
@@ -681,6 +702,15 @@ extern "C" int b200_gemm2_bf16(const void* A, const void* B, void* C, const void
     if (a_mn || b_mn || out_fp32 || !p.rope || (p.rope_hd % 8) || (p.rope_cols % 8)) return -8;
     return launch2<false, false, P_EPI_ROPE, __nv_bfloat16>(tmA, tmB, p, stream);
   }
+  if (epi & P_EPI_BIAS) {   // R = bias [N] bf16; nt, bf16 output
+    if (a_mn || b_mn || out_fp32 || !R || (reinterpret_cast<uintptr_t>(R) & 15) || (N % 8)) return -14;
+    if (epi == (P_EPI_ROPE | P_EPI_BIAS)) {
+      if (!p.rope || (p.rope_hd % 8) || (p.rope_cols % 8)) return -8;
+      return launch2<false, false, P_EPI_ROPE | P_EPI_BIAS, __nv_bfloat16>(tmA, tmB, p, stream);
+    }
+    if (epi == (P_EPI_STORE | P_EPI_BIAS)) return launch2<false, false, P_EPI_STORE | P_EPI_BIAS, __nv_bfloat16>(tmA, tmB, p, stream);
+    return -14;
+  }
   if (epi == P_EPI_PUSH) {   // wgrad (tn) only; every 8-element vector must stay inside one owner's slice
     if (!a_mn || !b_mn || out_fp32 || !p.push_bases || p.push_n <= 0 || (p.push_n % 8) || (p.push_off % 8) || (ldc % 8))
       return -9;
@@ -741,6 +771,15 @@ extern "C" int b200_gemm2_ag_bf16(const void* A, const void* B, void* C, const v
   if (epi == P_EPI_ROPE) {
     if (a_mn || b_mn || !p.rope || (p.rope_hd % 8) || (p.rope_cols % 8)) return -8;
     AGL(false, false, P_EPI_ROPE);
+  }
+  if (epi & P_EPI_BIAS) {   // R = bias [N] bf16; nt
+    if (a_mn || b_mn || !R || (reinterpret_cast<uintptr_t>(R) & 15) || (N % 8)) return -14;
+    if (epi == (P_EPI_ROPE | P_EPI_BIAS)) {
+      if (!p.rope || (p.rope_hd % 8) || (p.rope_cols % 8)) return -8;
+      AGL(false, false, P_EPI_ROPE | P_EPI_BIAS);
+    }
+    if (epi == (P_EPI_STORE | P_EPI_BIAS)) AGL(false, false, P_EPI_STORE | P_EPI_BIAS);
+    return -14;
   }
   if (!a_mn && !b_mn) {
     if (epi == P_EPI_SWIGLU) AGL(false, false, P_EPI_SWIGLU);

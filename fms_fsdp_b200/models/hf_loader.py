@@ -3,7 +3,8 @@
 the adapters of ``train_speculator_utils.py:526-569``):
 
 * Llama   -> ``LLaMA`` / ``EmbedLLaMA``: fuses q/k/v and gate/up, permutes q/k rows from HF's half-split RoPE layout back
-  to the FMS interleaved-pair layout (the inverse of ``fms_to_hf_llama._interleaved_to_halfsplit``);
+  to the FMS interleaved-pair layout (the inverse of ``fms_to_hf_llama._interleaved_to_halfsplit``); Qwen2 / Qwen2.5 (a
+  Llama block with q/k/v biases) loads the same way with ``qkv_bias=True``;
 * GPT-BigCode (multi-query attention, learned positions) -> ``EmbedGPTBigCode``;
 * Mixtral (Llama attention + top-k sparse MoE) -> ``EmbedMixtral``; both the hub format (``block_sparse_moe.experts.N.w1/w2/w3``)
   and the fused in-memory format of recent transformers (``mlp.experts.gate_up_proj / down_proj``)."""
@@ -20,7 +21,25 @@ from fms_fsdp_b200.models.llama import LLaMA, LLaMAConfig
 
 
 def _halfsplit_to_interleaved(w: torch.Tensor, nheads: int) -> torch.Tensor:
-    return w.view(nheads, 2, -1, w.size(1)).transpose(1, 2).reshape(*w.size())
+    """q / k projection rows (2-D weight) or entries (1-D bias) of each head from (i, i + hd/2) to (2i, 2i + 1) order."""
+    return w.view(nheads, 2, -1, *w.shape[1:]).transpose(1, 2).reshape(w.shape)
+
+
+def is_qwen2(hf_cfg: dict) -> bool:
+    """Qwen2 / Qwen2.5: Llama weight names and block, plus a bias on q, k and v (no ``attention_bias`` key says so)."""
+    return hf_cfg.get("model_type") == "qwen2" or "Qwen2ForCausalLM" in (hf_cfg.get("architectures") or [])
+
+
+def _sliding_window_in_use(hf_cfg: dict) -> bool:
+    window = hf_cfg.get("sliding_window")
+    if not window or window >= hf_cfg.get("max_position_embeddings", window):
+        return False
+    if hf_cfg.get("use_sliding_window") is False:          # Qwen2: the window is configured but switched off
+        return False
+    layer_types = hf_cfg.get("layer_types")
+    if layer_types and all(t == "full_attention" for t in layer_types):
+        return False
+    return True
 
 
 def _refuse_unsupported(hf_cfg: dict):
@@ -31,12 +50,12 @@ def _refuse_unsupported(hf_cfg: dict):
     if kind not in ("default", None, "llama3", "linear"):
         raise NotImplementedError(f"HF checkpoint uses rope scaling {kind!r}; plain RoPE, 'linear' and 'llama3' (Llama 3.1 / 3.2) "
                                   "are implemented, loading it would change the logits")
-    window = hf_cfg.get("sliding_window")
-    if window and window < hf_cfg.get("max_position_embeddings", window):
-        raise NotImplementedError(f"HF checkpoint uses sliding-window attention (window {window}); only full causal attention is "
-                                  "implemented")
+    if _sliding_window_in_use(hf_cfg):
+        raise NotImplementedError(f"HF checkpoint uses sliding-window attention (window {hf_cfg['sliding_window']}); only full "
+                                  "causal attention is implemented")
     if hf_cfg.get("attention_bias") or hf_cfg.get("mlp_bias"):
-        raise NotImplementedError("HF checkpoint has attention / MLP biases; the LLaMA blocks here are bias-free")
+        raise NotImplementedError("HF checkpoint has attention-output / MLP biases; the LLaMA blocks here carry a bias on the "
+                                  "q, k, v projection only (Qwen2)")
 
 
 def config_from_hf(hf_cfg: dict) -> LLaMAConfig:
@@ -51,7 +70,7 @@ def config_from_hf(hf_cfg: dict) -> LLaMAConfig:
         nheads=hf_cfg["num_attention_heads"], kvheads=hf_cfg.get("num_key_value_heads", 0) or 0,
         nlayers=hf_cfg["num_hidden_layers"], hidden_grow_factor=F / D, multiple_of=1,
         max_expected_seq_len=hf_cfg.get("max_position_embeddings", 4096), rope_theta=float(rope),
-        rope_scaling=rope_scaling)
+        rope_scaling=rope_scaling, qkv_bias=is_qwen2(hf_cfg))
 
 
 def _read_hf_tensors(model_path: str) -> Dict[str, torch.Tensor]:
@@ -69,7 +88,17 @@ def _read_hf_tensors(model_path: str) -> Dict[str, torch.Tensor]:
     return out
 
 
+def _refuse_unaccounted_biases(hf: Dict[str, torch.Tensor], cfg: LLaMAConfig):
+    """A bias tensor the config does not account for would be dropped and change the logits: stop instead."""
+    allowed = (".self_attn.q_proj.bias", ".self_attn.k_proj.bias", ".self_attn.v_proj.bias") if cfg.qkv_bias else ()
+    extra = sorted(k for k in hf if k.endswith(".bias") and not k.endswith(allowed))
+    if extra:
+        raise NotImplementedError(f"HF checkpoint carries bias tensors the model does not have ({', '.join(extra[:4])}"
+                                  f"{', ...' if len(extra) > 4 else ''}); loading it would drop them and change the logits")
+
+
 def convert_hf_state_dict(hf: Dict[str, torch.Tensor], cfg: LLaMAConfig) -> Dict[str, torch.Tensor]:
+    _refuse_unaccounted_biases(hf, cfg)
     sd = {"shared.emb.weight": hf["model.embed_tokens.weight"],
           "shared.head.weight": hf.get("lm_head.weight", hf["model.embed_tokens.weight"]),
           "dec_norm.weight": hf["model.norm.weight"]}
@@ -78,6 +107,10 @@ def convert_hf_state_dict(hf: Dict[str, torch.Tensor], cfg: LLaMAConfig) -> Dict
         q = _halfsplit_to_interleaved(hf[s + "self_attn.q_proj.weight"], cfg.nheads)
         k = _halfsplit_to_interleaved(hf[s + "self_attn.k_proj.weight"], cfg.kv_heads)
         sd[d + "attn.in_proj.qkv_fused.weight"] = torch.cat([q, k, hf[s + "self_attn.v_proj.weight"]], dim=0)
+        if cfg.qkv_bias:
+            sd[d + "attn.in_proj.qkv_fused.bias"] = torch.cat([
+                _halfsplit_to_interleaved(hf[s + "self_attn.q_proj.bias"], cfg.nheads),
+                _halfsplit_to_interleaved(hf[s + "self_attn.k_proj.bias"], cfg.kv_heads), hf[s + "self_attn.v_proj.bias"]])
         sd[d + "attn.dense.weight"] = hf[s + "self_attn.o_proj.weight"]
         sd[d + "ff_sub_layer.wg1_fused.weight"] = torch.cat([hf[s + "mlp.gate_proj.weight"], hf[s + "mlp.up_proj.weight"]], dim=0)
         sd[d + "ff_sub_layer.w2.weight"] = hf[s + "mlp.down_proj.weight"]
@@ -137,11 +170,12 @@ def load_hf_mixtral(model_path: str, model_cls, device="cpu", dtype=torch.bfloat
     with open(os.path.join(model_path, "config.json")) as f:
         c = json.load(f)
     cfg = config_from_hf(c)
+    hf = _read_hf_tensors(model_path)
+    _refuse_unaccounted_biases(hf, cfg)
     E, top_k = c["num_local_experts"], c.get("num_experts_per_tok", 2)
     with torch.device("meta"):
         model = model_cls(cfg, n_experts=E, top_k=top_k)
     model.to_empty(device=device)
-    hf = _read_hf_tensors(model_path)
     sd = {"shared.emb.weight": hf["model.embed_tokens.weight"],
           "shared.head.weight": hf.get("lm_head.weight", hf["model.embed_tokens.weight"]),
           "dec_norm.weight": hf["model.norm.weight"]}

@@ -47,6 +47,9 @@ class LLaMAConfig:
     # extension (not an fms field): HF-style frequency rescaling of long-context checkpoints, e.g. Llama 3.1
     # {"rope_type": "llama3", "factor": 8.0, "low_freq_factor": 1.0, "high_freq_factor": 4.0, "original_max_position_embeddings": 8192}
     rope_scaling: Optional[dict] = None
+    # extension (not an fms field): a bias on the fused q, k, v projection, added before RoPE (Qwen2 / Qwen2.5).
+    # State-dict key ``layers.N.attn.in_proj.qkv_fused.bias``; no bias on the output projection or the MLP.
+    qkv_bias: bool = False
 
     @property
     def hidden_dim(self) -> int:
@@ -63,15 +66,16 @@ class LLaMAConfig:
 
 
 class _Weight(nn.Module):
-    """A bias-free linear weight holder: keeps FMS's ``<name>.weight`` state-dict key."""
+    """A linear weight holder: keeps FMS's ``<name>.weight`` (and, with ``bias=True``, ``<name>.bias``) state-dict keys."""
 
-    def __init__(self, out_features: int, in_features: int, device=None, dtype=None):
+    def __init__(self, out_features: int, in_features: int, device=None, dtype=None, bias: bool = False):
         super().__init__()
         self.in_features, self.out_features = in_features, out_features
         self.weight = nn.Parameter(torch.empty(out_features, in_features, device=device, dtype=dtype))
+        self.bias = nn.Parameter(torch.empty(out_features, device=device, dtype=dtype)) if bias else None
 
     def forward(self, x, residual=None):
-        return ops.linear(x, self.weight, residual)
+        return ops.linear(x, self.weight, residual, bias=self.bias)
 
 
 class RMSNorm(nn.Module):
@@ -129,7 +133,7 @@ class _InProj(nn.Module):
         super().__init__()
         hd = cfg.head_dim
         self.splits = [cfg.nheads * hd, cfg.kv_heads * hd, cfg.kv_heads * hd]
-        self.qkv_fused = _Weight(sum(self.splits), cfg.emb_dim, device, dtype)
+        self.qkv_fused = _Weight(sum(self.splits), cfg.emb_dim, device, dtype, bias=getattr(cfg, "qkv_bias", False))
 
 
 class MultiHeadAttention(nn.Module):
@@ -143,6 +147,8 @@ class MultiHeadAttention(nn.Module):
     def reset_parameters(self):
         for w in (self.in_proj.qkv_fused.weight, self.dense.weight):
             nn.init.trunc_normal_(w, mean=0.0, std=0.02)
+        if self.in_proj.qkv_fused.bias is not None:
+            nn.init.zeros_(self.in_proj.qkv_fused.bias)
 
 
 class GatedLinearUnit(nn.Module):
@@ -202,7 +208,7 @@ class LLaMABlock(nn.Module):
         h, x = self.ln.fork(x)
         # projection + RoPE + attention: one node, RoPE fused into the GEMM / dq-dk epilogues
         ctx = ops.qkv_attention(h, a.in_proj.qkv_fused.weight, self._rot.table(x.device, S), a.nheads, a.kvheads,
-                                a.head_dim)
+                                a.head_dim, bias=a.in_proj.qkv_fused.bias)
         x = a.dense(ctx, residual=x)
         h, x = self.ff_ln.fork(x)
         ff = self.ff_sub_layer

@@ -98,7 +98,7 @@ def flush_ag_request(req=None):
                 _standalone_gather(r)
 
 
-def _try_fused_gather(a, b, layout, out, epi, residual) -> bool:
+def _try_fused_gather(a, b, layout, out, epi, residual, bias=None) -> bool:
     if not _AG_QUEUE:
         return False
     req = _AG_QUEUE[0]
@@ -124,7 +124,8 @@ def _try_fused_gather(a, b, layout, out, epi, residual) -> bool:
         take = max(_AG_CHUNK, (take + _AG_CHUNK - 1) // _AG_CHUNK * _AG_CHUNK)
         hi = min(end, begin + take)
     _C.gemm_ag(a, b, None if epi == 4 else out, _LAYOUT[layout], epi, residual, req["table"], req["full"], req["shard_bytes"], begin,
-               hi, req["world"], req["rank"], req["flags"], req["epoch"], bool(req["dependent"]))
+               hi, req["world"], req["rank"], req["flags"], req["epoch"], bool(req["dependent"]),
+               **({} if bias is None else {"bias": bias}))
     AG_STATS["carrier_gemms"] += 1
     if hi >= end:
         _AG_QUEUE.pop(0)
@@ -182,13 +183,25 @@ def _gemm_push(a, b, tgt: PushTarget):
 
 
 # ------------------------------------------------------------------------------------------ GEMM
-def gemm(a, b, layout="nt", out=None, accumulate=False, residual=None, out_dtype=None, rope=None):
+def _bias_fusable(a, b, layout, out, accumulate, residual, out_dtype, bias):
+    """Shapes the bias epilogue takes: CTA-pair nt GEMM with a bf16 output and a contiguous, 16-byte aligned bf16 bias."""
+    return (GEMM_IMPL == "tcgen05" and layout == "nt" and a.dtype == b.dtype == bias.dtype == torch.bfloat16
+            and residual is None and not accumulate and a.shape[0] >= 256 and _C.get_gemm_2cta()
+            and out_dtype in (None, torch.bfloat16) and (out is None or out.dtype == torch.bfloat16)
+            and bias.dim() == 1 and bias.numel() == b.shape[0] and bias.is_contiguous() and bias.data_ptr() % 16 == 0)
+
+
+def gemm(a, b, layout="nt", out=None, accumulate=False, residual=None, out_dtype=None, rope=None, bias=None):
     """``rope=(table [S, hd/2, 2] fp32, S, hd, H, KVH)``: rotary embedding of the q and k heads (the first
-    ``(H + KVH) * hd`` output columns) fused into the GEMM epilogue (QKV projection; nt layout)."""
+    ``(H + KVH) * hd`` output columns) fused into the GEMM epilogue (QKV projection; nt layout).
+    ``bias`` [N] bf16 (nt): added in fp32 to the accumulator before the RoPE rotation / store (P_EPI_BIAS)."""
     if isinstance(out, PushTarget):
-        if layout != "tn" or accumulate or residual is not None:
+        if layout != "tn" or accumulate or residual is not None or bias is not None:
             raise RuntimeError("the push epilogue is a plain tn (wgrad) store")
         return _gemm_push(a, b, out)
+    if bias is not None and not _bias_fusable(a, b, layout, out, accumulate, residual, out_dtype, bias):
+        return _fallback("gemm_bias").gemm(a, b, layout, out=out, accumulate=accumulate, residual=residual,
+                                           out_dtype=out_dtype, rope=rope, bias=bias)
     if rope is not None:
         M0 = a.shape[0]
         ok = (GEMM_IMPL == "tcgen05" and layout == "nt" and a.dtype == b.dtype == torch.bfloat16 and residual is None
@@ -196,7 +209,7 @@ def gemm(a, b, layout="nt", out=None, accumulate=False, residual=None, out_dtype
               and a.shape[1] % 8 == 0 and b.shape[0] % 8 == 0 and out_dtype in (None, torch.bfloat16)
               and (out is None or out.dtype == torch.bfloat16))
         if not ok:   # unfused: GEMM, then the in-place RoPE kernel
-            y = gemm(a, b, layout, out=out, accumulate=accumulate, residual=residual, out_dtype=out_dtype)
+            y = gemm(a, b, layout, out=out, accumulate=accumulate, residual=residual, out_dtype=out_dtype, bias=bias)
             table, S, hd, H, KVH = rope
             return rope_(y, table, S, H, KVH, hd)
     if GEMM_IMPL != "tcgen05" or a.dtype != torch.bfloat16 or b.dtype != torch.bfloat16:
@@ -209,7 +222,8 @@ def gemm(a, b, layout="nt", out=None, accumulate=False, residual=None, out_dtype
         M, N = a.shape[1], b.shape[1]
     K = a.shape[1] if layout != "tn" else a.shape[0]
     if (M % 8) or (N % 8) or (K % 8):
-        return _fallback("gemm").gemm(a, b, layout, out=out, accumulate=accumulate, residual=residual, out_dtype=out_dtype)
+        return _fallback("gemm").gemm(a, b, layout, out=out, accumulate=accumulate, residual=residual, out_dtype=out_dtype,
+                                      bias=bias)
     if a.stride(-1) != 1:
         a = a.contiguous()
     if b.stride(-1) != 1:
@@ -226,9 +240,20 @@ def gemm(a, b, layout="nt", out=None, accumulate=False, residual=None, out_dtype
     if rope is not None:
         epi = 3
         _C.set_gemm_rope(rope[0], int(rope[1]), int(rope[2]), int((rope[3] + rope[4]) * rope[2]))   # for the launch below
-    if _AG_QUEUE and _try_fused_gather(a, b, layout, out, epi, residual):
+    if _AG_QUEUE and _try_fused_gather(a, b, layout, out, epi, residual, bias):
         return out
-    _C.gemm(a, b, out, _LAYOUT[layout], epi, residual)
+    _C.gemm(a, b, out, _LAYOUT[layout], epi, residual, **({} if bias is None else {"bias": bias}))
+    return out
+
+
+def bias_grad(dy, out, accumulate=False):
+    """out[n] (+)= sum_m dy[m, n]: deterministic two-pass column sum (csrc/elementwise.cu bias_grad_*_kernel)."""
+    dy2 = dy.reshape(-1, dy.shape[-1])
+    if (dy2.dtype != torch.bfloat16 or dy2.shape[1] % 8 or out.dtype not in (torch.bfloat16, torch.float32)
+            or not out.is_contiguous() or out.numel() != dy2.shape[1]):
+        return _fallback("bias_grad").bias_grad(dy, out, accumulate)
+    dy2 = dy2 if dy2.is_contiguous() and dy2.data_ptr() % 16 == 0 else dy2.contiguous()
+    _C.bias_grad(dy2, out, bool(accumulate))
     return out
 
 

@@ -70,7 +70,7 @@ def _deliver_wgrad(w, compute):
 # ------------------------------------------------------------------------------------------ linear
 class _Linear(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, x, w, residual):
+    def forward(ctx, x, w, residual, bias=None):
         K = kernels_for(x)
         x2 = x.reshape(-1, x.shape[-1])
         r2 = None if residual is None else residual.reshape(-1, residual.shape[-1])
@@ -78,8 +78,8 @@ class _Linear(torch.autograd.Function):
         # allocate in the caller's shape: returning a view from a custom Function would forbid the
         # in-place RoPE that follows the QKV projection
         y = torch.empty(*x.shape[:-1], wd.shape[0], dtype=x.dtype, device=x.device)
-        K.gemm(x2, wd, "nt", out=y.view(-1, wd.shape[0]), residual=r2)
-        ctx.K, ctx.w, ctx.has_res = K, w, residual is not None
+        K.gemm(x2, wd, "nt", out=y.view(-1, wd.shape[0]), residual=r2, bias=None if bias is None else _wdata(bias))
+        ctx.K, ctx.w, ctx.b, ctx.has_res = K, w, bias, residual is not None
         ctx.save_for_backward(x)
         return y
 
@@ -97,7 +97,10 @@ class _Linear(torch.autograd.Function):
         dw = None
         if ctx.needs_input_grad[1]:
             dw = _deliver_wgrad(w, lambda out, acc: K.gemm(dy2, x2, "tn", out=out, accumulate=acc))
-        return dx, dw, (dy if ctx.has_res else None)
+        db = None
+        if ctx.b is not None and ctx.needs_input_grad[3]:
+            db = _deliver_wgrad(ctx.b, lambda out, acc: K.bias_grad(dy2, out, acc))
+        return dx, dw, (dy if ctx.has_res else None), db
 
 
 # ---- optional reduced-precision forward GEMMs (default "bf16"; "fp8" is opt-in and never used for the headline metric)
@@ -121,7 +124,7 @@ class _LinearFP8(torch.autograd.Function):
     backward recipe).  Activations and weights stay bf16 in memory."""
 
     @staticmethod
-    def forward(ctx, x, w, residual):
+    def forward(ctx, x, w, residual, bias=None):
         K = kernels_for(x)
         x2 = x.reshape(-1, x.shape[-1])
         wd = _wdata(w)
@@ -129,20 +132,22 @@ class _LinearFP8(torch.autograd.Function):
         wq, sw = K.quant_rowwise_e4m3(wd if wd.is_contiguous() else wd.contiguous())
         y = torch.empty(*x.shape[:-1], wd.shape[0], dtype=x.dtype, device=x.device)
         K.gemm_fp8(xq, wq, sx, sw, out=y.view(-1, wd.shape[0]))
+        if bias is not None:   # unfused: the fp8 path is opt-in and its epilogue carries the scales
+            y += _wdata(bias)
         if residual is not None:
             y += residual
-        ctx.K, ctx.w, ctx.has_res = K, w, residual is not None
+        ctx.K, ctx.w, ctx.b, ctx.has_res = K, w, bias, residual is not None
         ctx.save_for_backward(x)
         return y
 
     backward = _Linear.backward
 
 
-def linear(x, w, residual: Optional[torch.Tensor] = None):
-    """y = x @ w^T (+ residual, fused in the GEMM epilogue)."""
+def linear(x, w, residual: Optional[torch.Tensor] = None, bias: Optional[torch.Tensor] = None):
+    """y = x @ w^T (+ bias [N]) (+ residual), bias and residual fused in the GEMM epilogue."""
     if _GEMM_PRECISION == "fp8" and x.dtype == torch.bfloat16 and x.shape[-1] % 16 == 0:
-        return _LinearFP8.apply(x, w, residual)
-    return _Linear.apply(x, w, residual)
+        return _LinearFP8.apply(x, w, residual, bias)
+    return _Linear.apply(x, w, residual, bias)
 
 
 # ----------------------------------------------------------------------------------------- rmsnorm
@@ -294,13 +299,13 @@ class _QKVAttention(torch.autograd.Function):
     (SURVEY.md K1-K3; reference path: fms MultiHeadAttention.in_proj -> RotaryEmbedding.adjusted_qk -> SDPA)."""
 
     @staticmethod
-    def forward(ctx, h, w, table, S, H, KVH, hd, scale):
+    def forward(ctx, h, w, table, S, H, KVH, hd, scale, bias=None):
         K = kernels_for(h)
         B = h.shape[0]
         h2 = h.reshape(-1, h.shape[-1])
-        qkv = K.gemm(h2, _wdata(w), "nt", rope=(table, S, hd, H, KVH))
+        qkv = K.gemm(h2, _wdata(w), "nt", rope=(table, S, hd, H, KVH), bias=None if bias is None else _wdata(bias))
         o, lse = K.attn_fwd(qkv, B, S, H, KVH, hd, scale)
-        ctx.K, ctx.w, ctx.args = K, w, (B, S, H, KVH, hd, scale)
+        ctx.K, ctx.w, ctx.b, ctx.args = K, w, bias, (B, S, H, KVH, hd, scale)
         ctx.save_for_backward(h, qkv, o, lse, table)
         return o.view(B, S, H * hd)
 
@@ -316,16 +321,21 @@ class _QKVAttention(torch.autograd.Function):
         dw = None
         if ctx.needs_input_grad[1]:
             dw = _deliver_wgrad(w, lambda out, acc: K.gemm(dqkv, h2, "tn", out=out, accumulate=acc))
-        return dh, dw, None, None, None, None, None, None
+        db = None
+        if ctx.b is not None and ctx.needs_input_grad[8]:   # the bias sits before RoPE: dL/db = column sums of dqkv
+            db = _deliver_wgrad(ctx.b, lambda out, acc: K.bias_grad(dqkv, out, acc))
+        return dh, dw, None, None, None, None, None, None, db
 
 
-def qkv_attention(h, w, table, nheads, kvheads, head_dim, scale=None):
-    """attention(rope(h @ w^T)) for a fused [(H + 2 KVH) * hd, D] projection weight; h: [B, S, D]."""
+def qkv_attention(h, w, table, nheads, kvheads, head_dim, scale=None, bias=None):
+    """attention(rope(h @ w^T + bias)) for a fused [(H + 2 KVH) * hd, D] projection weight and optional [(H + 2 KVH) * hd]
+    bias (Qwen2); h: [B, S, D]."""
     S = h.shape[1]
     scale = (head_dim ** -0.5) if scale is None else scale
     if _GEMM_PRECISION == "fp8":     # fp8 projection, then the stand-alone RoPE kernel and attention
-        return attention(rope_(linear(h, w), table, S, nheads, kvheads, head_dim), nheads, kvheads, head_dim, scale)
-    return _QKVAttention.apply(h, w, table, S, nheads, kvheads, head_dim, scale)
+        return attention(rope_(linear(h, w, bias=bias), table, S, nheads, kvheads, head_dim), nheads, kvheads, head_dim,
+                         scale)
+    return _QKVAttention.apply(h, w, table, S, nheads, kvheads, head_dim, scale, bias)
 
 
 def attention(qkv, nheads, kvheads, head_dim, scale=None):

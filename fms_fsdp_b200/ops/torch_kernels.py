@@ -20,12 +20,17 @@ NAME = "torch"
 # GEMM family.  layout: "nt": C[M,N] = A[M,K] B[N,K]^T ; "nn": C[M,N] = A[M,K] B[K,N] ;
 #                        "tn": C[M,N] = A[K,M]^T B[K,N].  fp32 accumulate, output dtype of `out`/a.
 # ----------------------------------------------------------------------------------------------
-def gemm(a, b, layout="nt", out=None, accumulate=False, residual=None, out_dtype=None, rope=None):
+def gemm(a, b, layout="nt", out=None, accumulate=False, residual=None, out_dtype=None, rope=None, bias=None):
+    """``bias`` [N] (nt only): added to the product before the RoPE rotation / residual."""
     if rope is not None:   # (table, S, head_dim, H, KVH): RoPE on the q and k heads of a fused QKV product
-        y = gemm(a, b, layout, out=out, accumulate=accumulate, residual=residual, out_dtype=out_dtype)
+        y = gemm(a, b, layout, out=out, accumulate=accumulate, residual=residual, out_dtype=out_dtype, bias=bias)
         table, S, hd, H, KVH = rope
         return rope_(y, table, S, H, KVH, hd)
-    if layout == "nt":
+    if bias is not None:
+        if layout != "nt":
+            raise ValueError("bias: nt layout only")
+        c = torch.addmm(bias.to(a.dtype), a, b.t())
+    elif layout == "nt":
         c = a @ b.t()
     elif layout == "nn":
         c = a @ b
@@ -41,6 +46,16 @@ def gemm(a, b, layout="nt", out=None, accumulate=False, residual=None, out_dtype
         out.add_(c.to(out.dtype))
     else:
         out.copy_(c)
+    return out
+
+
+def bias_grad(dy, out, accumulate=False):
+    """out[n] (+)= sum_m dy[m, n] with fp32 accumulation (gradient of a bias added to every row of a GEMM output)."""
+    s = dy.reshape(-1, dy.shape[-1]).float().sum(0)
+    if accumulate:
+        out.add_(s.to(out.dtype))
+    else:
+        out.copy_(s)
     return out
 
 

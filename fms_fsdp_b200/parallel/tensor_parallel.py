@@ -29,6 +29,10 @@ def _slice_llama_attention(blk, c, tp: int, r: int):
     H, KV = c.nheads // tp, c.kv_heads // tp
     q, k, v = torch.split(blk.attn.in_proj.qkv_fused.weight.data, [c.nheads * hd, c.kv_heads * hd, c.kv_heads * hd], dim=0)
     blk.attn.in_proj.qkv_fused.weight.data = torch.cat([_rows(q, r, H * hd), _rows(k, r, KV * hd), _rows(v, r, KV * hd)])
+    bias = blk.attn.in_proj.qkv_fused.bias
+    if bias is not None:   # qkv_bias (Qwen2): sliced by heads exactly like the weight rows
+        q, k, v = torch.split(bias.data, [c.nheads * hd, c.kv_heads * hd, c.kv_heads * hd])
+        bias.data = torch.cat([_rows(q, r, H * hd), _rows(k, r, KV * hd), _rows(v, r, KV * hd)])
     blk.attn.dense.weight.data = _cols(blk.attn.dense.weight.data, r, H * hd)
     blk.attn.nheads, blk.attn.kvheads = H, KV
 

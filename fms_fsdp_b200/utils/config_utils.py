@@ -63,6 +63,13 @@ _LLAMA_ZOO: Dict[str, Dict[str, Any]] = {
     # --- extensions (BASELINE.json config #1; plumbing / CPU-gloo tests)
     "llama2_tiny": dict(src_vocab_size=1024, emb_dim=256, nheads=4, kvheads=4, nlayers=2,
                         hidden_grow_factor=8 / 3, multiple_of=64, max_expected_seq_len=512),
+    # --- Qwen2 family: Llama block + q/k/v projection bias (HF Qwen2ForCausalLM).  qwen2.5_7b follows the published
+    # config.json (not checked against a downloaded file; hf_to_fms_llama.py --model_variant compares on first use)
+    "qwen2.5_7b": dict(src_vocab_size=152064, emb_dim=3584, nheads=28, kvheads=4, nlayers=28,
+                       hidden_grow_factor=18944 / 3584, norm_eps=1e-6, max_expected_seq_len=32768,
+                       rope_theta=1000000.0, qkv_bias=True),
+    "qwen2_tiny": dict(src_vocab_size=1024, emb_dim=256, nheads=4, kvheads=2, nlayers=2, hidden_grow_factor=2,
+                       multiple_of=64, norm_eps=1e-6, max_expected_seq_len=512, rope_theta=1000000.0, qkv_bias=True),
 }
 
 _MAMBA_ZOO: Dict[str, Dict[str, Any]] = {

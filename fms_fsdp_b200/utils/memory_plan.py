@@ -73,6 +73,8 @@ def plan_llama(model_variant: str, gpus: int = 1, sharding_strategy: str = "fsdp
     T = batch_size * seq_length
 
     block_params = (c.nheads * hd + 2 * kvd) * D + D * c.nheads * hd + 2 * F * D + D * F + 2 * D
+    if c.qkv_bias:
+        block_params += c.nheads * hd + 2 * kvd
     root_params = 2 * V * D + D
     n_params = L * block_params + root_params
 

@@ -1,4 +1,5 @@
-"""Export a sharded training checkpoint to a HuggingFace ``LlamaForCausalLM`` directory
+"""Export a sharded training checkpoint to a HuggingFace ``LlamaForCausalLM`` directory (``Qwen2ForCausalLM`` for a model
+with ``qkv_bias``)
 (CLI parity with reference ``fms_to_hf_llama.py:133-171``):
 
     python fms_to_hf_llama.py --model_variant llama2_7b --nocompiled --load_path <step_N_ckp> \
@@ -20,16 +21,17 @@ from fms_fsdp_b200.utils.config_utils import get_model_config
 
 
 def _interleaved_to_halfsplit(w: torch.Tensor, nheads: int) -> torch.Tensor:
-    """rows [h, (pair, 2)] -> [h, (2, pair)]: (x0,x1,x2,x3,..) -> (x0,x2,..,x1,x3,..) per head."""
-    return w.view(nheads, -1, 2, w.size(1)).transpose(1, 2).reshape(*w.size())
+    """rows [h, (pair, 2)] -> [h, (2, pair)]: (x0,x1,x2,x3,..) -> (x0,x2,..,x1,x3,..) per head (2-D weight or 1-D bias)."""
+    return w.view(nheads, -1, 2, *w.shape[1:]).transpose(1, 2).reshape(w.shape)
 
 
 def convert_to_hf(model: LLaMA, model_variant: str, is_old_fms: bool = False):
     """``is_old_fms`` is kept for the reference's signature; this repo's LLaMA is always fused, pre-fusion checkpoints are
     fused when they are read (``load_dcp_into``)."""
-    from transformers import LlamaConfig, LlamaForCausalLM
+    from transformers import LlamaConfig, LlamaForCausalLM, Qwen2Config, Qwen2ForCausalLM
 
     c = model.config
+    qwen2 = getattr(c, "qkv_bias", False)
     rope_theta = c.rope_theta
     if c.ntk_scaling:
         alpha = model.rot_emb._alpha(c.max_expected_seq_len)
@@ -38,13 +40,17 @@ def convert_to_hf(model: LLaMA, model_variant: str, is_old_fms: bool = False):
         vocab_size=c.src_vocab_size, hidden_size=c.emb_dim, rms_norm_eps=c.norm_eps, num_attention_heads=c.nheads,
         num_key_value_heads=c.kv_heads, num_hidden_layers=c.nlayers, intermediate_size=c.hidden_dim,
         pad_token_id=None if c.pad_id == -1 else c.pad_id, max_position_embeddings=c.max_expected_seq_len,
-        rope_theta=rope_theta, tie_word_embeddings=False, attention_bias=False, mlp_bias=False,
+        rope_theta=rope_theta, tie_word_embeddings=False,
     )
+    if not qwen2:
+        kw.update(attention_bias=False, mlp_bias=False)
+    else:   # Qwen2: biased q/k/v, full attention (the window is configured but switched off)
+        kw.update(use_sliding_window=False, sliding_window=None)
     if "llama3" in model_variant:
         kw.update(bos_token_id=128000, eos_token_id=128001)
     if getattr(c, "rope_scaling", None):          # long-context frequency rescaling travels with the export
         kw["rope_scaling"] = dict(c.rope_scaling)
-    hf = LlamaForCausalLM(LlamaConfig(**kw))
+    hf = Qwen2ForCausalLM(Qwen2Config(**kw)) if qwen2 else LlamaForCausalLM(LlamaConfig(**kw))
     sd = model.state_dict()
     hd = c.head_dim
     with torch.no_grad():
@@ -56,6 +62,12 @@ def convert_to_hf(model: LLaMA, model_variant: str, is_old_fms: bool = False):
             layer.self_attn.q_proj.weight.copy_(_interleaved_to_halfsplit(q, c.nheads))
             layer.self_attn.k_proj.weight.copy_(_interleaved_to_halfsplit(k, c.kv_heads))
             layer.self_attn.v_proj.weight.copy_(v)
+            if qwen2:
+                qb, kb, vb = torch.split(sd[p + "attn.in_proj.qkv_fused.bias"],
+                                         [c.nheads * hd, c.kv_heads * hd, c.kv_heads * hd])
+                layer.self_attn.q_proj.bias.copy_(_interleaved_to_halfsplit(qb, c.nheads))
+                layer.self_attn.k_proj.bias.copy_(_interleaved_to_halfsplit(kb, c.kv_heads))
+                layer.self_attn.v_proj.bias.copy_(vb)
             layer.self_attn.o_proj.weight.copy_(sd[p + "attn.dense.weight"])
             fused = sd[p + "ff_sub_layer.wg1_fused.weight"]
             wg, w1 = torch.split(fused, [fused.size(0) // 2, fused.size(0) // 2], dim=0)
@@ -143,7 +155,7 @@ def main(model_variant, compiled=False, is_old_fms=False, load_path=None, save_p
     model.to_empty(device="cpu")
     print(f"Reading state dict from {load_path}")
     load_dcp_into(model, load_path, compiled, is_old_fms)
-    print("Converting to HF Llama...")
+    print("Converting to HF Qwen2..." if cfg.qkv_bias else "Converting to HF Llama...")
     hf = convert_to_hf(model, model_variant, is_old_fms)
     hf.save_pretrained(save_path)
     print(f"Model saving at {save_path}")

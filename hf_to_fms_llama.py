@@ -1,6 +1,6 @@
-"""Import a HuggingFace ``LlamaForCausalLM`` directory as a single-file model checkpoint for this trainer -- the inverse of
-``fms_to_hf_llama.py`` (the reference has only the export direction; continued pre-training / fine-tuning from public
-weights needs the way back):
+"""Import a HuggingFace ``LlamaForCausalLM`` (or ``Qwen2ForCausalLM``) directory as a single-file model checkpoint for this
+trainer -- the inverse of ``fms_to_hf_llama.py`` (the reference has only the export direction; continued pre-training /
+fine-tuning from public weights needs the way back):
 
     python hf_to_fms_llama.py --hf_path <hf dir> --save_path llama.pth [--model_variant llama2_7b]
     torchrun ... main_training_llama.py --model_variant=llama2_7b --ckpt_load_path=llama.pth ...
@@ -20,7 +20,8 @@ from fms_fsdp_b200.models.hf_loader import _read_hf_tensors, config_from_hf, con
 from fms_fsdp_b200.utils.cli import run
 from fms_fsdp_b200.utils.config_utils import get_model_config
 
-_CHECKED = ("src_vocab_size", "emb_dim", "nheads", "kv_heads", "nlayers", "hidden_dim", "rope_theta", "rope_scaling")
+_CHECKED = ("src_vocab_size", "emb_dim", "nheads", "kv_heads", "nlayers", "hidden_dim", "rope_theta", "rope_scaling",
+            "qkv_bias")
 
 
 def main(hf_path: str, save_path: str, model_variant: str = "", dtype: str = "bf16"):
